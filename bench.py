@@ -2,7 +2,7 @@
 """bench.py — headline benchmark of the B200 hot path (BASELINE.json: DLRM & TwoTower fwd samples/s).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
-                    [--workload all|dlrm|dlrm-sharded|twotower|dcn|dlrm-train] [--batch B]
+                    [--workload all|dlrm|dlrm-sharded|twotower|dcn|dlrm-train] [--batch B] [--dump-outputs DIR]
 
 Headline workload = BASELINE.json configs[1]: mm.DLRMModel, Criteo shape (26 cat, 13 dense, emb 64,
 bundled cardinalities = 45.6 M rows / 11.7 GB of tables), batch 65 536, README MLP dims.
@@ -26,6 +26,9 @@ The default `--workload all` adds to the same line:
       protocol timed beside it.
 `--impl reference` times the CPU restatement alone on the SAME 65 536-sample step (TensorFlow is not
 installable: no network).  `--workload dlrm|twotower|dcn|dlrm-sharded` print a line for that workload only.
+`--dump-outputs DIR` writes, after the timed steps, what each timed path computed in its last timed step as
+DIR/<name>.npy (float32, rank 0; a fixed, seeded row sample where an output is too large).  Inputs, tables and
+weights are seeded, so two builds run with the same arguments can be compared output for output.
 """
 from __future__ import annotations
 
@@ -161,6 +164,36 @@ def dlrm_bytes_per_sample(T=26, D=64, id_bytes_total=104, P=64):
 
 NCU_FUSED_SUMMARY = "profiles/r02_ncu_fused_operand.txt"  # `ncu --set full` summary of THIS round's dominant kernel
 
+DUMP_LIMIT_BYTES = 64 << 20  # all of --dump-outputs together
+DUMP_SAMPLE_BYTES = 16 << 20  # an output larger than this is dumped as a seeded row sample of about this size
+DUMP_SEED = 0
+
+
+def last_output(pf):
+    """Device output of the last step submitted to the pipeline `pf`."""
+    return pf.output((pf.n - 1) % len(pf.slots))
+
+
+def sample_rows(t, n=None):
+    """A fixed, seeded sample of the rows of the 2-D tensor `t` (of `n` rows, or of about DUMP_SAMPLE_BYTES), in row order."""
+    import torch
+
+    if n is None:
+        n = DUMP_SAMPLE_BYTES // (4 * max(1, t[0].numel()))
+    n = max(1, min(int(n), t.shape[0]))
+    idx = np.sort(np.random.default_rng(DUMP_SEED).choice(t.shape[0], size=n, replace=False))
+    return t[torch.from_numpy(idx).to(t.device)]
+
+
+def write_dumps(out_dir, arrays):
+    total = sum(a.nbytes for a in arrays.values())
+    if total > DUMP_LIMIT_BYTES:
+        raise RuntimeError(f"--dump-outputs: {total} bytes exceed the {DUMP_LIMIT_BYTES}-byte limit")
+    d = Path(out_dir)
+    d.mkdir(parents=True, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(d / f"{name}.npy", a)
+
 
 def cpu_baseline_dlrm(model, feats_host, sample_rows, threads):
     """CPU restatement (oracle/oracle_torch.py) on `sample_rows` samples of the same workload, with
@@ -193,6 +226,13 @@ class Ctx:
     def __init__(self, args, mm, datasets, ops, dev, rank, local_rank, world):
         self.args, self.mm, self.datasets, self.ops = args, mm, datasets, ops
         self.dev, self.rank, self.local_rank, self.world = dev, rank, local_rank, world
+        self.dumping = bool(args.dump_outputs) and rank == 0
+        self.dumps = {}
+
+    def dump(self, name, t):
+        """Keep a float32 host copy of an output of a timed path for --dump-outputs (nothing when not dumping)."""
+        if self.dumping:
+            self.dumps[name] = t.detach().float().cpu().numpy()
 
     def barrier(self):
         import torch
@@ -351,6 +391,7 @@ def dlrm_record(ctx):
     assert torch.equal(model(devs[1]), pf.output(0)), "pipelined replay diverges from model.__call__"
 
     elapsed_ms, clocks = timed_replay(ctx, pf, packed_dev, args.steps, args.warmup)
+    ctx.dump("dlrm_predictions", last_output(pf))
     launches = cf.launches_per_replay * args.steps
     serial_ms = timed_serial(cf, packed_dev, args.steps)
 
@@ -450,6 +491,8 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--pipeline-depth", type=int, default=3,
                     help="graph instances / streams of model.pipeline (3: one more pinned H2D in flight than 2)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what each timed path computed in its last timed step as DIR/<name>.npy (rank 0)")
     args = ap.parse_args()
     if args.warmup < 3:
         args.warmup = 3
@@ -483,6 +526,8 @@ def main():
     ctx = Ctx(args, mm, datasets, ops, dev, rank, local_rank, world)
 
     def finish(line):
+        if ctx.dumping:
+            write_dumps(args.dump_outputs, ctx.dumps)
         if rank == 0:
             print(json.dumps(line))
         if dist.is_initialized():
@@ -646,6 +691,7 @@ def sharded_record(ctx):
         graph_ok = int(torch.equal(cf.replay(), want))
         pf = model.pipeline(hbs[0], depth=args.pipeline_depth)
         elapsed_ms, clocks = timed_replay(ctx, pf, packed_dev, steps, args.warmup)
+        ctx.dump(f"sharded_{label}_predictions", last_output(pf))
         serial_ms = timed_serial(cf, packed_dev, steps)
         # the fused lookup + interaction kernel alone
         body = model.body
@@ -808,6 +854,15 @@ def train_record(ctx):
     clocks = sampler.stop()
     ms = t0.elapsed_time(t1)
     loss_end = float(tr.loss.item())
+    if ctx.dumping:
+        # the loss of the last timed step and the variables it left: every Dense variable, and the embedding rows of a
+        # seeded sample of that step's samples (rows it updated)
+        ctx.dump("dlrm_train_loss", tr.loss)
+        ctx.dump("dlrm_train_dense_variables", tr.arena.w)
+        last = hosts[(steps - 1) % n_bufs]
+        pos = np.sort(np.random.default_rng(DUMP_SEED).choice(B, size=min(256, B), replace=False))
+        ctx.dump("dlrm_train_embedding_rows_sample",
+                 torch.stack([t.table[torch.from_numpy(last[f].reshape(-1)[pos].astype(np.int64)).to(dev)] for f, t in zip(tr.feats, tr.tables)]))
     # e2e: pinned host batch -> H2D -> graph -> loss to the host
     loss_host = torch.zeros(1, dtype=torch.float32, pin_memory=True)
 
@@ -943,6 +998,11 @@ def secondary_record(ctx, kind):
     cf = model.compile(hbs[0], **call_kwargs)
     pf = model.pipeline(hbs[0], depth=2, **call_kwargs)
     elapsed_ms, clocks = timed_replay(ctx, pf, packed_dev, steps, args.warmup)
+    if kind == "twotower":  # (B, 1+B) logits: 1 GB at B = 16 384
+        if ctx.dumping:
+            ctx.dump("twotower_logits_row_sample", sample_rows(last_output(pf)))
+    else:
+        ctx.dump("dcn_predictions", last_output(pf))
     serial_ms = timed_serial(cf, packed_dev, steps)
 
     # dominant kernel, one launch per CUDA-event pair
@@ -1018,6 +1078,7 @@ def secondary_record(ctx, kind):
             cf2 = model.compile(hbs[0], **kw)
             pf2 = model.pipeline(hbs[0], depth=2, **kw)
             el2, _ = timed_replay(ctx, pf2, packed_dev, steps, args.warmup)
+            ctx.dump("twotower_fused_loss_stats", last_output(pf2))
             ser2 = timed_serial(cf2, packed_dev, steps)
             e2e2, res2 = timed_e2e(ctx, pf2, hbs, e2e_steps, 2)
             el2, e2e2 = ctx.max_over_ranks(el2, e2e2)
@@ -1066,12 +1127,13 @@ def reference_arm(args, mm, datasets, cores):
     rng = np.random.default_rng(4321)
     cat = schema.select_by_tag(mm.Tags.CATEGORICAL)
     # host tables: random rows are touched uniformly, so the table content is irrelevant to the
-    # timing; sizes (rows x 64 fp32) are the real ones, filled by a cheap generator
+    # timing; sizes (rows x 64 fp32) are the real ones, filled by a cheap seeded generator
+    gen = torch.Generator().manual_seed(4321)
     tables = {}
     for c in cat:
         rows = c.int_domain.max + 1
         t = torch.empty((rows, 64), dtype=torch.float32)
-        t.uniform_(-0.05, 0.05)
+        t.uniform_(-0.05, 0.05, generator=gen)
         tables[c.name] = t
     f2t = {c.name: c.name for c in cat}
 
@@ -1099,15 +1161,13 @@ def reference_arm(args, mm, datasets, cores):
     cores = pick_threads(run, cores)
     for _ in range(max(1, min(args.warmup, 3))):
         run()
-    steps = args.steps
+    done = args.steps
     t0 = time.perf_counter()
-    done = 0
-    for _ in range(steps):
-        run()
-        done += 1
-        if time.perf_counter() - t0 > 120.0:
-            break
+    for _ in range(done):
+        out = run()
     dt = time.perf_counter() - t0
+    if args.dump_outputs:
+        write_dumps(args.dump_outputs, {"reference_predictions": out.float().numpy()})
     value = sample * done / dt
     line = {
         "impl": "reference",
